@@ -10,8 +10,12 @@ configurations, each with its own roofline / e2e / cpu_baseline (see build_workl
 
   python bench.py --gpus N --steps K --warmup W [--config cfgK]            # our engine
   python bench.py --impl reference --gpus N --steps K ... [--config cfgK]  # CPU restatement of the reference
+  python bench.py ... --dump-outputs DIR     # also write the last timed step's outputs as DIR/<name>.npy
 
-Prints ONE JSON line (see the contract in the task statement).
+Inputs (theta, point sets) come from fixed seeds, so two builds run with the same arguments can be compared through
+their dumped outputs.
+
+Prints ONE JSON line on stdout.
 """
 from __future__ import annotations
 
@@ -251,7 +255,9 @@ def run_reference(args, rank: int, world: int):
     n_pts = sum(s.shape[1] for s in s2[:n_pde])
     for _ in range(max(1, min(args.warmup, 2))):
         cpu_reference_eval(cfg, theta, s2, cores, 1, q2)
-    L, times, _ = cpu_reference_eval(cfg, theta, s2, cores, args.steps, q2)
+    L, times, G = cpu_reference_eval(cfg, theta, s2, cores, args.steps, q2)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"loss": np.array([L]), "grad": G})
     total = float(np.sum(times))
     val = n_pts * args.steps / total
     line = {
@@ -268,6 +274,14 @@ def run_reference(args, rank: int, world: int):
         "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir: str, arrays):
+    """Write each array as out_dir/<name>.npy in the dtype it was computed in (float32 on the GPU, float64 on the CPU
+    arm), so that two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a))
 
 
 def run_ours(args, rank: int, local_rank: int, world: int):
@@ -339,6 +353,11 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     t_total = float(ms.sum()) * 1e-3
     loss_val = float(total_d.item())
     grad_h = grad_d.cpu().numpy().astype(np.float64)
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results, before the measurements below overwrite the buffers (the gradient and the
+        # losses are already summed over the ranks, so rank 0 holds what every rank holds)
+        dump_outputs(args.dump_outputs, {"loss": total_d.cpu().numpy(), "term_losses": terms_d.cpu().numpy(),
+                                         "grad": grad_d.cpu().numpy()})
 
     # ---- main-kernel duration (for the roofline), events inside the library around the fused kernel ----
     eng.set_timing(True)
@@ -475,6 +494,8 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-alt-modes", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, term_losses, grad) as DIR/<name>.npy")
     args = ap.parse_args()
     # stdout carries exactly one JSON line: NCCL's version banner / debug output (printed to stdout when NCCL_DEBUG is
     # set in the environment) goes to stderr instead

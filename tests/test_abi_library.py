@@ -29,8 +29,11 @@ def test_library_exports_every_declared_symbol():
 
 def test_library_is_in_tree_and_sm100a():
     assert os.path.dirname(npde.LIB_PATH) == os.path.join(ROOT, "neuralpde.jl_b200", "lib")
+    import shutil
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", npde.LIB_PATH], capture_output=True, text=True).stdout
+    # the toolkit's bin directory need not be on PATH; build.py falls back to the default install for nvcc likewise
+    cuobjdump = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
+    out = subprocess.run([cuobjdump, "-lelf", npde.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
 
 
